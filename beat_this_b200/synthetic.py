@@ -16,6 +16,7 @@ from __future__ import annotations
 
 import math
 import os
+import tempfile
 from collections import OrderedDict
 
 import numpy as np
@@ -137,6 +138,12 @@ def make_checkpoint(name: str = "final0", seed: int = 0) -> dict:
         "datamodule_hyper_parameters": {},
         "pytorch-lightning_version": "2.1.0",
     }
+
+
+def cache_dir() -> str:
+    """Where tests and benchmarks keep the checkpoints and audio they generate: $BT_TEST_CACHE, else a directory of
+    the calling user's own under the system's temporary directory (another user's copy there is not writable)."""
+    return os.environ.get("BT_TEST_CACHE") or os.path.join(tempfile.gettempdir(), f"beat_this_b200_cache_{os.getuid()}")
 
 
 def write_checkpoint(path: str, name: str = "final0", seed: int = 0) -> str:

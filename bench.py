@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus 1 --steps K ...  # the UNMODIFIED reference (baseline/_ref) on host cores
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --config 3|4|5 ...                       # the other BASELINE configs (files / --dbn / ragged)
+    python bench.py --dump-outputs DIR ...                   # also write the last timed step's outputs as DIR/*.npy
 
 One "step" = one pass of the hot path over one batch of `--batch` synthetic 30 s clips per GPU (BASELINE config 2:
 Audio2Frames final0, batch 64; the minimal peak picker is included so that the step is audio -> beats).  Prints ONE
@@ -48,9 +49,11 @@ if ROOT not in sys.path:
 import numpy as np
 import torch
 
+from beat_this_b200.synthetic import cache_dir
+
 SR = 22050
 METRIC = "clips/sec (30 s audio->beats, final0)"
-CACHE = os.environ.get("BT_TEST_CACHE", "/tmp/beat_this_b200_cache")
+CACHE = cache_dir()
 REF_DIR = os.path.join(ROOT, "baseline", "_ref")
 
 
@@ -353,6 +356,38 @@ def reduce_sum(world, dev, v):
     return int(t[0])
 
 
+DUMP_LIMIT_BYTES = 63 << 20  # array data; with the .npy headers the files stay below 64 MB
+
+
+def dump_outputs(out_dir: str, beat: torch.Tensor, down: torch.Tensor, times: list) -> None:
+    """Write what one step of the timed path returned, so that two builds can be compared output for output:
+    beat_logits / downbeat_logits (float32, [clips, frames]; every clip of the batch has the same length),
+    beat_times / downbeat_times (float64, all clips concatenated) with beat_counts / downbeat_counts per clip, and
+    clip_index, the clips of the batch they belong to.  Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of
+    clips is written."""
+    n = len(times)
+    beat = beat.view(n, -1).cpu().numpy()
+    down = down.view(n, -1).cpu().numpy()
+    size = np.asarray([beat.shape[1] * 8 + (len(b) + len(d) + 3) * 8 for b, d in times])
+    keep = np.arange(n)
+    if size.sum() > DUMP_LIMIT_BYTES:
+        order = np.random.default_rng(0).permutation(n)
+        keep = np.sort(order[np.cumsum(size[order]) <= DUMP_LIMIT_BYTES])
+    out = {
+        "beat_logits": beat[keep],
+        "downbeat_logits": down[keep],
+        "beat_times": np.concatenate([times[i][0] for i in keep]).astype(np.float64),
+        "downbeat_times": np.concatenate([times[i][1] for i in keep]).astype(np.float64),
+        "beat_counts": np.asarray([len(times[i][0]) for i in keep], dtype=np.float64),
+        "downbeat_counts": np.asarray([len(times[i][1]) for i in keep], dtype=np.float64),
+        "clip_index": keep.astype(np.float64),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), arr)
+    print(f"outputs of the last timed step ({len(keep)} of {n} clips) written to {out_dir}", file=sys.stderr)
+
+
 def run_ours(args, rank, world, local):
     import torch.distributed as dist
 
@@ -382,17 +417,18 @@ def run_ours(args, rank, world, local):
 
     def step_device():
         beat, down, f = eng.audio2frames_cat(audio_dev, so)
-        return eng.peakpick_cat(beat, down, f)
+        return beat, down, eng.peakpick_cat(beat, down, f)
 
     def timed_device_steps():
+        """(elapsed ms, what the last step returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(args.steps):
-            step_device()
+            out = step_device()
         e1.record()
         barrier()
-        return e0.elapsed_time(e1)
+        return e0.elapsed_time(e1), out
 
     # ---- device-resident timing (no per-kernel events) ----------------------------------------------------
     for _ in range(args.warmup):
@@ -400,13 +436,13 @@ def run_ours(args, rank, world, local):
     sampler = ClockSampler(local)
     sampler.start()
     l0 = eng.launches
-    ms = timed_device_steps()
+    ms, last_step = timed_device_steps()
     launches = eng.launches - l0
     clocks = sampler.stop()
     # ---- second timed pass with one CUDA event per launch: per-kernel times for the roofline ---------------
     eng.profile_reset()
     eng.profile_enable(True)
-    ms_prof = timed_device_steps()
+    ms_prof, _ = timed_device_steps()
     eng.profile_enable(False)
     prof = eng.profile_results()
     # ---- end to end through the reference-signature API ---------------------------------------------------
@@ -432,6 +468,8 @@ def run_ours(args, rank, world, local):
     launches = reduce_sum(world, dev, launches)
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last_step)
     peaks, peak_src = load_peaks()
     total_clips = args.batch * world
     value = total_clips * args.steps / (ms / 1000.0)
@@ -624,7 +662,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-reference", action="store_true")
     ap.add_argument("--ref-clips-per-step", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="config 2: write the logits and beat / downbeat times of the "
+                    "last timed step (rank 0) as .npy files to DIR")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "ours" or args.config != 2):
+        ap.error("--dump-outputs writes the outputs of the config 2 timed path (--impl ours)")
     from beat_this_b200.distributed import init_from_env
 
     if args.impl == "reference":

@@ -8,7 +8,6 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-CACHE = os.environ.get("BT_TEST_CACHE", "/tmp/beat_this_b200_cache")
 
 
 def pytest_configure(config):
@@ -22,7 +21,7 @@ def pytest_configure(config):
 def ckpt_path(name: str, seed: int = 0) -> str:
     from beat_this_b200 import synthetic
 
-    return synthetic.write_checkpoint(os.path.join(CACHE, f"{name}_s{seed}.ckpt"), name, seed)
+    return synthetic.write_checkpoint(os.path.join(synthetic.cache_dir(), f"{name}_s{seed}.ckpt"), name, seed)
 
 
 @pytest.fixture(scope="session")

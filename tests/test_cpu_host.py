@@ -85,16 +85,25 @@ def test_packed_parameters_reproduce_the_oracle(name):
     assert all(np.array_equal(back[k], packed[k]) for k in packed)
 
 
-def test_checkpoint_layout_roundtrip(small0_ckpt):
-    from beat_this_b200.inference import load_checkpoint
+def test_checkpoint_layout_roundtrip(small0_ckpt, monkeypatch):
+    from beat_this_b200.inference import CHECKPOINT_URL, load_checkpoint
 
     ck = load_checkpoint(small0_ckpt)
     assert set(ck) >= {"state_dict", "hyper_parameters"}
     assert all(k.startswith("model.") for k in ck["state_dict"])
     assert len(ck["state_dict"]) == 166
     assert sum(v.numel() for v in ck["state_dict"].values()) == 2101357  # SURVEY.md App. B (small0)
+    # a path that is not a file falls through to the URL path; the download is stubbed to fail as it does offline
+    urls = []
+
+    def no_network(url, **kw):
+        urls.append(url)
+        raise OSError("no network")
+
+    monkeypatch.setattr(torch.hub, "load_state_dict_from_url", no_network)
     with pytest.raises(ValueError):
-        load_checkpoint("/nonexistent/dir/nothing-here")  # falls through to the URL path, no network -> ValueError
+        load_checkpoint("/nonexistent/dir/nothing-here")
+    assert urls == [f"{CHECKPOINT_URL}//nonexistent/dir/nothing-here.ckpt"]
 
 
 def test_api_surface_matches_reference_names():

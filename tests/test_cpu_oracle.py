@@ -1,14 +1,12 @@
 """CPU tests (no GPU): the oracle restatement against the golden fixtures generated from the
-UNMODIFIED reference (oracle/make_golden.py), and -- when /root/reference is present (the
-build container) -- directly against the reference modules."""
+UNMODIFIED reference (oracle/make_golden*.py)."""
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN, ROOT
+from conftest import GOLDEN
 
 from beat_this_b200 import synthetic
 from oracle import beat_this_oracle as O
@@ -93,25 +91,24 @@ def test_model_golden_final0_short_clip(final0_ckpt):
     assert np.array_equal(bt, g["final0_clip1_beat_times"]) and np.array_equal(dt, g["final0_clip1_down_times"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/beat_this"), reason="reference tree only exists in the build container")
 def test_oracle_against_live_reference(small0_ckpt):
-    sys.path.insert(0, os.path.join(ROOT, "oracle", "shims"))
-    sys.path.insert(0, "/root/reference")
-    import beat_this.inference as ref_inf  # noqa: E402
+    """The reference's BeatThis module and split_piece, as recorded by oracle/make_golden_forward.py."""
+    from oracle.make_golden_forward import FORWARD_SEED, SPLIT_LENGTHS
 
-    model = ref_inf.load_model(small0_ckpt, "cpu")  # strict load: the synthetic .ckpt has the reference layout
+    g = np.load(os.path.join(GOLDEN, "reference_forward.npz"))
     sd = O.strip_prefix(torch.load(small0_ckpt, weights_only=True)["state_dict"])
-    torch.manual_seed(4)
+    assert abs(synthetic.tensor_checksum(sd) - float(g["small0_ckpt_sum"])) < 1e-6 * abs(float(g["small0_ckpt_sum"]))
+    # the reference's load_model loads strictly: the synthetic .ckpt must have its layout, name for name
+    assert {k: str(tuple(v.shape)) for k, v in sd.items()} == dict(zip(g["state_keys"].tolist(), g["state_shapes"].tolist()))
+    torch.manual_seed(FORWARD_SEED)
     x = torch.rand(2, 100, 128) * 7
     with torch.inference_mode():
-        ref = model(x)
         b, d = O.forward(sd, x)
         eb, ed = O.forward(sd, x, explicit=True)
-    assert (ref["beat"] - b).abs().max() < 1e-4 and (ref["downbeat"] - d).abs().max() < 1e-4
+    assert np.abs(g["beat"] - b.numpy()).max() < 1e-4 and np.abs(g["downbeat"] - d.numpy()).max() < 1e-4
     assert (eb - b).abs().max() < 1e-4
-    for T in (1, 1488, 1489, 3001):
-        _, starts = ref_inf.split_piece(torch.zeros(T, 1), 1500, 6, True)
-        assert np.array_equal(starts, O.split_starts(T))
+    for T in SPLIT_LENGTHS:
+        assert np.array_equal(g[f"starts_{T}"], O.split_starts(T))
 
 
 # ------------------------------------------------------------------------------------ resampler

@@ -14,7 +14,7 @@ from beat_this_b200.inference import Audio2Beats
 
 n_clips = int(sys.argv[1]) if len(sys.argv) > 1 else 8
 steps = int(sys.argv[2]) if len(sys.argv) > 2 else 2
-ckpt = synthetic.write_checkpoint("/tmp/beat_this_b200_cache/final0_s0.ckpt", "final0", 0)
+ckpt = synthetic.write_checkpoint(os.path.join(synthetic.cache_dir(), "final0_s0.ckpt"), "final0", 0)
 a2b = Audio2Beats(ckpt, "cuda:0", float16=True)
 a2b.model.engine.set_wave_chunks(2 * n_clips)
 clips = [synthetic.synth_clip(2000 + (i % 4), 30.0).astype("float32") for i in range(n_clips)]
